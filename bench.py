@@ -5,7 +5,7 @@ One "step" = one pass of the hot path over one batch of synthetic input: forward
 InterpolatingAdjoint gradient of the L2 trajectory-matching loss, summed over the ensemble (+ the sum over ranks of
 [grad_theta; loss] when N_gpus > 1, fused into the final reduction kernel over NVLink peer memory).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config lv|seir|fkpp|hjb]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config lv|seir|fkpp|hjb] [--dump-outputs DIR]
 
 --config lv (default, BASELINE config 2): 2->32->32->2 tanh chain, Glorot theta (seed 1), u0 ~ U(0.2,1) x U(2,5), 30 fixed
   Tsit5 steps of 0.1, states saved at every step, fp32.  The headline `value` is WEAK scaling (65 536 trajectories per GPU);
@@ -15,6 +15,9 @@ InterpolatingAdjoint gradient of the L2 trajectory-matching loss, summed over th
 --config hjb (config 5): highdim_pde/lambaem.jl's NNPDENS solve (d = 100, hls = 110, 20 Euler-Maruyama steps), 10 000 paths per GPU
   and iteration, fp64; a step = one iteration (forward paths + reverse sweep + ADAM); metric = paths/s.
 Under torchrun one rank per GPU.  Rank 0 prints ONE JSON line.
+--dump-outputs DIR: rank 0 writes what the last timed step returned as DIR/<name>.npy (lv / seir / fkpp: out[n_save, d, N] of its
+  shard, grad_theta, loss; hjb: theta after the update, loss, u0 on 1 GPU or grad_theta, loss on several), so that two builds can be
+  compared output for output on the same seeded inputs.
 """
 import argparse
 import json
@@ -181,6 +184,22 @@ class FKPP:
 
 CONFIGS = {"lv": LV, "seir": SEIR, "fkpp": FKPP}
 HOST = None
+DUMP_BYTES = 60_000_000     # data written by --dump-outputs: keeps the files, headers included, under 64 MB
+
+
+def write_outputs(dirname, **arrays):
+    """--dump-outputs: the host arrays as dirname/<name>.npy.  `out` (trajectories on the last axis) is cut to a fixed, seeded sample of
+    trajectories when the files would pass DUMP_BYTES in all."""
+    os.makedirs(dirname, exist_ok=True)
+    out = arrays.get("out")
+    room = DUMP_BYTES - sum(v.nbytes for k, v in arrays.items() if k != "out")
+    if out is not None and out.nbytes > room:
+        n = out.shape[-1]
+        keep = np.sort(np.random.default_rng(0).choice(n, room // (out.nbytes // n), replace=False))
+        arrays["out"] = np.ascontiguousarray(out[..., keep])
+    for k, v in arrays.items():
+        np.save(os.path.join(dirname, k + ".npy"), v)
+    print(f"[bench] wrote {', '.join(f'{k}{list(v.shape)}' for k, v in arrays.items())} to {dirname}", file=sys.stderr)
 
 
 class ClockSampler:
@@ -241,7 +260,7 @@ def reference_arm(a, cfg):
     for _ in range(max(1, min(a.warmup, 2))):
         k = min(n, 1024)
         cpu_pass(cfg, theta, np.ascontiguousarray(u0[:, :k]), np.ascontiguousarray(y[:, :, :k]), cores)
-    times = [cpu_pass(cfg, theta, u0, y, cores) for _ in range(max(3, a.steps))]
+    times = [cpu_pass(cfg, theta, u0, y, cores) for _ in range(a.steps)]
     med = float(np.median(times))
     value = n / med
     same = (cfg is LV and n == N_PER_GPU)
@@ -300,7 +319,7 @@ def main_hjb(a):
         ms = min(m, 2000)
         bo.loss_and_grad(theta, d, hls, np.zeros(d), 1.0, n_steps, 200, 1)
         times = []
-        for i in range(max(3, min(a.steps, 5))):
+        for i in range(a.steps):
             t0 = time.perf_counter(); bo.loss_and_grad(theta, d, hls, np.zeros(d), 1.0, n_steps, ms, 1 + i); times.append(time.perf_counter() - t0)
         v = ms / float(np.median(times))
         print(json.dumps({"impl": "reference", "metric": metric, "value": v, "unit": unit, "n_gpus": a.gpus, "steps": len(times), "warmup": 1,
@@ -340,7 +359,7 @@ def main_hjb(a):
     if world == 1:
         s.train_adam(opt, m, max(a.warmup, 3), seed0=1)
         torch.cuda.synchronize()
-        s.train_adam(opt, m, a.steps, seed0=100)
+        hist = s.train_adam(opt, m, a.steps, seed0=100)
         total_ms = s.last_train_ms()
         timing = "CUDA events on the handle's stream around the K iterations (1 direct launch + K-1 replays of one CUDA graph)"
     else:
@@ -357,6 +376,9 @@ def main_hjb(a):
         total_ms = float(t)
         timing = "host clock around K synchronous iterations (each ends in a stream synchronize), max over ranks"
     value = world * m * a.steps / (total_ms * 1e-3)
+    if a.dump_outputs and rank == 0:
+        last = {"loss": hist[0][-1:], "u0": hist[1][-1:]} if world == 1 else {"grad_theta": g_all[:s.P], "loss": g_all[s.P:]}
+        write_outputs(a.dump_outputs, theta=s.get_params(), **{k: v.cpu().numpy() for k, v in last.items()})
 
     # end to end through the host-buffer call a script makes per optimiser iteration: theta in from host, loss + gradient back to host
     th_h = np.ascontiguousarray(s.get_params())
@@ -462,7 +484,12 @@ def main():
     ap.add_argument("--cpu-sample", type=int, default=0, help="trajectories in the in-line CPU baseline sample (0 = auto)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-strong", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned to DIR/<name>.npy (GPU arm)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's results; the reference arm keeps none")
     global HOST
     if a.config == "hjb":
         HOST = host_cores()
@@ -571,6 +598,8 @@ def main():
     weak = Shard(n, seed=rank)                       # every rank owns a different shard of the (world * n) ensemble
     tw = timed(weak)
     value = world * n * a.steps / (tw["total_ms"] * 1e-3)
+    if a.dump_outputs and rank == 0:                 # before the phases below reuse the shard's buffers
+        write_outputs(a.dump_outputs, out=weak.out_d.cpu().numpy(), grad_theta=weak.buf[:P].cpu().numpy(), loss=weak.buf[P:].cpu().numpy())
 
     # ---- the metric's literal batch: 65 536 trajectories in total, sharded over the ranks (strong scaling) ----
     strong = None

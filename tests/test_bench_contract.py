@@ -50,10 +50,32 @@ def test_reference_arm_live(extra):
     assert out.returncode == 0, out.stderr[-2000:]
     j = json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][-1])
     _check_common(j)
-    assert j["impl"] == "reference" and j["value"] > 0
+    assert j["impl"] == "reference" and j["value"] > 0 and j["steps"] == 3
     assert j["e2e"]["value"] == j["value"] and j["e2e"]["h2d_bytes_per_step"] == 0 and j["e2e"]["d2h_bytes_per_step"] == 0
     b = j["cpu_baseline"]
     assert b["kind"] == "port" and b["value"] == j["value"] and b["cores"] >= 1 and isinstance(b["sample"], str)
+
+
+@pytest.mark.gpu
+def test_dump_outputs_hold_the_last_timed_step(tmp_path, O):
+    """--dump-outputs writes what the timed step returns -- the saved states, loss and grad_theta of the seeded LV ensemble -- and they
+    agree with the CPU oracle on the same inputs."""
+    import numpy as np
+    from helpers import glorot_theta, synthetic_ensemble
+    n = 1024
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "1", "--n-per-gpu", str(n),
+                          "--no-strong", "--no-cpu-baseline", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600)
+    assert out.returncode == 0, out.stderr[-2000:]
+    assert json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][-1])["steps"] == 2
+    got = {k: np.load(tmp_path / f"{k}.npy") for k in ("out", "grad_theta", "loss")}
+    assert {k: (v.shape, v.dtype) for k, v in got.items()} == {"out": ((31, 2, n), np.float32), "grad_theta": ((1218,), np.float32),
+                                                                 "loss": ((1,), np.float32)}
+    theta = glorot_theta((2, 32, 32, 2), seed=1)
+    u0, y = synthetic_ensemble(n, seed=0)
+    l64, g64, _, out64 = O.ensemble_loss_grad(O.lv_model(), theta.astype(np.float64), u0, y, np.ones(2), 0.1, 30, want_out=True)
+    assert np.all(np.abs(got["out"] - out64) <= 3e-4 * (1 + np.abs(out64)))
+    assert abs(got["loss"][0] - l64) <= 1e-4 * abs(l64)
+    assert np.linalg.norm(got["grad_theta"] - g64) <= 2e-3 * np.linalg.norm(g64)
 
 
 def test_reference_arm_other_ranks_exit_quietly():

@@ -83,8 +83,8 @@ def test_sciml_train_bfgs_and_callback_halt():
     A = torch.tensor([[3.0, 0.5], [0.5, 1.0]])
     b = torch.tensor([1.0, -2.0])
 
-    def loss(th):
-        return 0.5 * th @ (A @ th) - b @ th
+    def loss(th):   # sciml_train puts a numpy theta on the current CUDA device when there is one
+        return 0.5 * th @ (A.to(th.device) @ th) - b.to(th.device) @ th
     res = ude.sciml_train(loss, np.zeros(2, np.float32), ude.BFGS(initial_stepnorm=0.01), maxiters=200)
     sol = torch.linalg.solve(A, b)
     assert torch.allclose(res.minimizer.cpu(), sol, atol=1e-4)

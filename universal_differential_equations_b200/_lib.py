@@ -6,6 +6,7 @@ the calls raise.  Nothing here imports the CPU oracle.
 """
 import ctypes as C
 import os
+import shutil
 import subprocess
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -77,10 +78,16 @@ class B200UDEError(RuntimeError):
         self.code = code
 
 
+def _nvcc():
+    """$NVCC, else nvcc on PATH, else the toolkit's under $CUDA_HOME or the default install location (a user's PATH may lack it)."""
+    home = os.environ.get("CUDA_HOME") or os.environ.get("CUDA_PATH") or "/usr/local/cuda"
+    return os.environ.get("NVCC") or shutil.which("nvcc") or os.path.join(home, "bin", "nvcc")
+
+
 def build(verbose=False):
     """Compile csrc/ for sm_100a in-tree (nvcc cross-compiles without a GPU)."""
     jobs = str(min(8, os.cpu_count() or 1))
-    subprocess.check_call(["make", "-C", CSRC, "-j", jobs] + ([] if verbose else ["-s"]))
+    subprocess.check_call(["make", "-C", CSRC, "-j", jobs, f"NVCC={_nvcc()}"] + ([] if verbose else ["-s"]))
     return SO_PATH
 
 
