@@ -235,6 +235,54 @@ int32_t b200ude_peer_detach(b200ude_handle *h);
 int32_t b200ude_adjoint_l2_allreduce(b200ude_handle *h, const void *data, void *loss, void *grad_theta, void *grad_u0,
                                      void *stream);
 
+/* BATCHED INDEPENDENT TRAININGS  (replaces the loop of LotkaVolterra/run_loops.jl:55-62, which calls recover_dynamics
+ * (loop_recoveries.jl) once per noisy data set, one run after another: each run trains its own theta with ADAM(0.1) on its own
+ * data and u0).  A batch handle holds M "members", each with its own theta, gradient and ADAM moments, one trajectory per member;
+ * nothing is shared between members (no ensemble sum, no shared optimiser state).  A member's results are bitwise independent of M,
+ * of its position in the batch and of the other members, and repeated calls are bitwise identical.
+ * Descriptor: b200ude_desc as for b200ude_create, restricted to the LV model with the 2-5-5-5-2 chain (identity output layer, per-layer
+ * activations, n_prefix 0..2 trainable rates: scenario 1 / the loop, scenario 2, Hudson Bay), fp32, fixed-step Tsit5, either sensealg;
+ * max_trajectories is the member capacity.  Anything else is B200UDE_EUNSUPPORTED; the descriptor is validated before the device is
+ * probed.  There is no CPU fallback.
+ * Layouts: u0 [d][M], data / out [n_save][d][M], status / loss [M], loss_history [iters][M] (member-fastest);
+ * theta / grad [M][P]: each member's flat theta is contiguous in the reference's own order (a Julia P x M matrix, one column per run).
+ * All arrays except a HOST theta are DEVICE pointers.  The physics constants, loss weights and activations of a batch handle sit in the
+ * constant bank of the batch kernels (not shared with the other families): work of two batch handles with different descriptors on one
+ * device must be stream-ordered; a batch handle may run concurrently with any non-batch handle. */
+typedef struct b200ude_batch_handle b200ude_batch_handle;
+int32_t b200ude_batch_create(const b200ude_desc *desc, b200ude_batch_handle **out);
+void b200ude_batch_destroy(b200ude_batch_handle *h);
+/* message of the last error on this handle (h may be NULL: last b200ude_batch_create error of the calling thread) */
+const char *b200ude_batch_last_error(const b200ude_batch_handle *h);
+/* P, the length of one member's theta (87 + n_prefix) */
+size_t b200ude_batch_num_params(const b200ude_batch_handle *h);
+/* theta [M][P] from host or device memory -> the handle's thetas of members 0..M-1; zeroes every member's ADAM moments and step
+ * count and makes theta its best theta so far (with loss +inf).  Later calls may use any M' <= M of these members: each member
+ * keeps its own step count, so a member trained by fewer calls than another continues from its own state. */
+int32_t b200ude_batch_set_params(b200ude_batch_handle *h, const void *theta, size_t M, int32_t mem, void *stream);
+/* the current thetas of members 0..M-1 -> theta [M][P] (host: synchronises the stream; device: asynchronous) */
+int32_t b200ude_batch_get_params(b200ude_batch_handle *h, void *theta, size_t M, int32_t mem, void *stream);
+/* FORWARD of every member at its own theta from its own u0: out [n_save][d][M], status [M] (may be NULL; B200UDE_TRAJ_NONFINITE when
+ * the final state is not finite). */
+int32_t b200ude_batch_forward(b200ude_batch_handle *h, const void *u0, size_t M, void *out, int32_t *status, void *stream);
+/* per-member fused L2 loss  loss[n] = sum_i sum_k w_k (u_n - data_n)^2  and its gradient grad [M][P] with respect to the member's own
+ * theta (the desc's sensealg), status [M] or NULL (non-finite state, loss or gradient).  What a host-side batched optimiser calls. */
+int32_t b200ude_batch_loss_gradient(b200ude_batch_handle *h, const void *u0, const void *data, size_t M, void *loss, void *grad,
+                                    int32_t *status, void *stream);
+/* `iters` ADAM iterations of every member in ONE launch (forward, fused-L2 adjoint, the member's loss, Flux.ADAM with its own moments;
+ * options and loss as b200ude_train_adam: L = loss_scale * L_data + l2_reg * sum theta[n_prefix:]^2).  loss_history [iters][M] or
+ * NULL: slot (i, n) = member n's loss at its pre-update theta of iteration i.  A member whose state, loss or gradient turns non-finite
+ * stops there: status[n] = B200UDE_TRAJ_NONFINITE, its theta and moments keep their last finite values, its remaining loss slots are
+ * NaN, and every other member is unaffected.  status [M] may be NULL.  Successive calls continue every member's moments and its own
+ * step count (advanced only by the member's own updates: a stopped member's stays where it stopped).  Each member also keeps the
+ * best pre-update theta since set_params and its loss, as sciml_train does (b200ude_batch_get_best). */
+int32_t b200ude_batch_train_adam(b200ude_batch_handle *h, const b200ude_adam *opt, const void *u0, const void *data, size_t M,
+                                 int32_t iters, void *loss_history, int32_t *status, void *stream);
+/* every member's best theta since set_params -> theta [M][P] and its loss -> loss [M] (the lowest recorded pre-update loss of
+ * b200ude_batch_train_adam; +inf and the set_params theta when there was no finite one) -- what sciml_train returns as its minimizer.
+ * Host: synchronises the stream; device: asynchronous. */
+int32_t b200ude_batch_get_best(b200ude_batch_handle *h, void *theta, void *loss, size_t M, int32_t mem, void *stream);
+
 /* SELF-TEST of a device building block (no reference counterpart): y[i] = the kernels' tanh (1 - 2 / (1 + 2^(2 log2(e) x)) with one
  * reciprocal per four values, the variant the warp-collective LV kernels use) for n device floats; the parity tests compare it
  * with tanh in fp64.  device = CUDA ordinal. */

@@ -7,9 +7,9 @@ mirror of the reference's call surface (sciml.py).  See DESIGN.md.
 """
 from . import _lib  # noqa: F401
 from .sciml import (  # noqa: F401
-    ADAM, BFGS, Chain, Dense, EnsembleProblem, FastChain, FastDense, FisherKPPUDE, ForwardDiffSensitivity,
-    InterpolatingAdjoint, LotkaVolterraUDE, NeuralODE, ODEProblem, SEIRExposureUDE, SEIRNeuralODE, ReverseDiffVJP, RKC2, ROCK2, Tsit5, UDESolver, Vern7,
-    concrete_solve, identity, initial_params, rbf, remake, sciml_train, sciml_train_l2, solve, tanh,
+    ADAM, BFGS, BatchTrainResult, Chain, Dense, EnsembleProblem, FastChain, FastDense, FisherKPPUDE, ForwardDiffSensitivity,
+    InterpolatingAdjoint, LotkaVolterraUDE, NeuralODE, ODEProblem, SEIRExposureUDE, SEIRNeuralODE, ReverseDiffVJP, RKC2, ROCK2, Tsit5, UDEBatchSolver, UDESolver,
+    Vern7, concrete_solve, identity, initial_params, rbf, remake, sciml_train, sciml_train_batch, sciml_train_l2, solve, tanh,
 )
 from . import pde  # noqa: F401
 from . import jld2  # noqa: F401

@@ -33,6 +33,9 @@ EXPORTS = [
     "b200ude_peer_export", "b200ude_peer_attach", "b200ude_peer_detach", "b200ude_adjoint_l2_allreduce", "b200ude_selftest_tanh",
     "b200ude_bsde_create", "b200ude_bsde_destroy", "b200ude_bsde_last_error", "b200ude_bsde_num_params", "b200ude_bsde_set_params",
     "b200ude_bsde_get_params", "b200ude_bsde_loss_gradient", "b200ude_bsde_train_adam", "b200ude_bsde_adam_step", "b200ude_bsde_last_train_ms", "b200ude_bsde_last_sweep_ms",
+    "b200ude_batch_create", "b200ude_batch_destroy", "b200ude_batch_last_error", "b200ude_batch_num_params", "b200ude_batch_set_params",
+    "b200ude_batch_get_params", "b200ude_batch_forward", "b200ude_batch_loss_gradient", "b200ude_batch_train_adam",
+    "b200ude_batch_get_best",
 ]
 PEER_HANDLE_BYTES = 64
 
@@ -168,6 +171,25 @@ def lib():
     L.b200ude_bsde_last_sweep_ms.argtypes = [vp, C.POINTER(C.c_double)]
     L.b200ude_bsde_adam_step.restype = i32
     L.b200ude_bsde_adam_step.argtypes = [vp, C.POINTER(Adam), vp]
+    L.b200ude_batch_create.restype = i32
+    L.b200ude_batch_create.argtypes = [C.POINTER(Desc), C.POINTER(vp)]
+    L.b200ude_batch_destroy.restype = None
+    L.b200ude_batch_destroy.argtypes = [vp]
+    L.b200ude_batch_last_error.restype = C.c_char_p
+    L.b200ude_batch_last_error.argtypes = [vp]
+    L.b200ude_batch_num_params.restype = sz
+    L.b200ude_batch_num_params.argtypes = [vp]
+    for f in ("b200ude_batch_set_params", "b200ude_batch_get_params"):
+        getattr(L, f).restype = i32
+        getattr(L, f).argtypes = [vp, vp, sz, i32, vp]
+    L.b200ude_batch_forward.restype = i32
+    L.b200ude_batch_forward.argtypes = [vp, vp, sz, vp, vp, vp]
+    L.b200ude_batch_loss_gradient.restype = i32
+    L.b200ude_batch_loss_gradient.argtypes = [vp, vp, vp, sz, vp, vp, vp, vp]
+    L.b200ude_batch_train_adam.restype = i32
+    L.b200ude_batch_train_adam.argtypes = [vp, C.POINTER(Adam), vp, vp, sz, i32, vp, vp, vp]
+    L.b200ude_batch_get_best.restype = i32
+    L.b200ude_batch_get_best.argtypes = [vp, vp, vp, sz, i32, vp]
     if L.b200ude_version() != ABI_VERSION:
         raise RuntimeError("libb200ude.so ABI version mismatch")
     _lib = L
@@ -183,4 +205,10 @@ def check_bsde(handle, rc):
 def check(handle, rc):
     if rc != 0:
         msg = lib().b200ude_last_error(handle)
+        raise B200UDEError(rc, msg.decode() if msg else "")
+
+
+def check_batch(handle, rc):
+    if rc != 0:
+        msg = lib().b200ude_batch_last_error(handle)
         raise B200UDEError(rc, msg.decode() if msg else "")

@@ -11,6 +11,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <limits>
 #include <new>
 #include <algorithm>
 #include <atomic>
@@ -104,17 +105,38 @@ struct b200ude_handle {
     std::string err;
 };
 
+// ---- batched independent trainings (b200ude_batch_*, k_batch.cu) ---------------------------------------------------------------
+struct b200ude_batch_handle {
+    b200ude_desc desc;
+    int P = 0, n_save = 0;
+    size_t cap = 0;        // member capacity
+    size_t members = 0;    // members whose theta set_params has stored
+    ConstTables tab;
+    float *d_theta = nullptr;             // [cap][P]
+    float *d_m = nullptr, *d_v = nullptr; // [P][cap]
+    float *d_ustep = nullptr, *d_dense = nullptr, *d_out = nullptr;   // forward record [..][D][M], saved-state scratch
+    int32_t *d_t = nullptr;               // [cap] ADAM steps each member has taken since set_params
+    float *d_best = nullptr;              // [cap][P] each member's best pre-update theta since set_params
+    float *d_best_loss = nullptr;         // [cap] its loss (+inf: no finite loss yet)
+    std::string err;
+};
+
 namespace {
 
-int32_t fail(b200ude_handle *h, int32_t code, const char *fmt, ...)
+// where a failure's message goes: the handle's own string, or the calling thread's last create() error
+std::string &err_of(b200ude_handle *h) { return h ? h->err : g_create_error; }
+std::string &err_of(b200ude_batch_handle *h) { return h ? h->err : g_create_error; }
+std::string &err_of(std::nullptr_t) { return g_create_error; }
+
+template <class H>
+int32_t fail(H h, int32_t code, const char *fmt, ...)
 {
     char buf[512];
     va_list ap;
     va_start(ap, fmt);
     vsnprintf(buf, sizeof(buf), fmt, ap);
     va_end(ap);
-    if (h) h->err = buf;
-    else g_create_error = buf;
+    err_of(h) = buf;
     return code;
 }
 
@@ -534,6 +556,37 @@ int32_t do_adjoint64(b200ude_handle *h, bool l2, const double *cot, double *loss
 int32_t f64_unsupported(b200ude_handle *h, const char *what)
 {
     return fail(h, B200UDE_EUNSUPPORTED, "%s: not available for B200UDE_F64 handles (device-pointer forward / adjoint entry points only)", what);
+}
+
+}  // namespace
+
+namespace {
+
+// the checks every batch call shares; fills the fields of p that do not depend on the call
+int32_t batch_prepare(b200ude_batch_handle *h, size_t M, const void *u0, int mode, BatchParams &p)
+{
+    CUDA_TRY(h, cudaSetDevice(h->desc.device));
+    if (h->members == 0) return fail(h, B200UDE_ESTATE, "batch: b200ude_batch_set_params has not been called");
+    if (M == 0 || M > h->members) return fail(h, B200UDE_EINVAL, "batch: M=%zu outside (0, members set=%zu]", M, h->members);
+    if (!u0) return fail(h, B200UDE_EINVAL, "batch: null u0");
+    p = BatchParams{};
+    p.u0 = (const float *)u0; p.out = h->d_out; p.theta = h->d_theta; p.m = h->d_m; p.v = h->d_v;
+    p.ustep = h->d_ustep; p.dense = h->d_dense;
+    p.t = h->d_t; p.best = h->d_best; p.best_loss = h->d_best_loss;
+    p.M = (int)M; p.ldm = (int)h->cap; p.n_steps = h->desc.n_steps; p.save_every = h->desc.save_every; p.mode = mode; p.iters = 1;
+    p.dt = (float)h->desc.dt;
+    return B200UDE_OK;
+}
+
+__global__ void fill_kernel(float *a, float v, size_t n)
+{
+    for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) a[i] = v;
+}
+
+int32_t batch_launch(b200ude_batch_handle *h, const BatchParams &p, cudaStream_t st)
+{
+    CUDA_TRY(h, launch_batch(h->desc.n_prefix, h->desc.sensealg == B200UDE_DISCRETE_ADJOINT, h->tab, p, st));
+    return B200UDE_OK;
 }
 
 }  // namespace
@@ -1029,6 +1082,185 @@ int32_t b200ude_selftest_tanh(int32_t device, const void *x, void *y, size_t n, 
     if (!x || !y || n == 0) return fail(nullptr, B200UDE_EINVAL, "selftest_tanh: null pointer or n == 0");
     CUDA_TRY(nullptr, cudaSetDevice(device));
     CUDA_TRY(nullptr, launch_tanh_selftest((const float *)x, (float *)y, n, (cudaStream_t)stream));
+    return B200UDE_OK;
+}
+
+// ---- batched independent trainings -------------------------------------------------------------------------------------------
+int32_t b200ude_batch_create(const b200ude_desc *d, b200ude_batch_handle **out)
+{
+    if (!d || !out) return fail(nullptr, B200UDE_EINVAL, "batch_create: null argument");
+    *out = nullptr;
+    if (d->struct_size != sizeof(b200ude_desc))
+        return fail(nullptr, B200UDE_EINVAL, "batch_create: struct_size %u != %zu (ABI mismatch)", d->struct_size, sizeof(b200ude_desc));
+    if (d->dtype != B200UDE_F32 && d->dtype != B200UDE_F64) return fail(nullptr, B200UDE_EINVAL, "batch_create: unknown dtype %d", d->dtype);
+    if (d->n_layers < 1 || d->n_layers > B200UDE_MAX_LAYERS) return fail(nullptr, B200UDE_EINVAL, "batch_create: n_layers=%d out of range", d->n_layers);
+    if (d->solver != B200UDE_TSIT5 && d->solver != B200UDE_VERN7 && d->solver != B200UDE_RKC2)
+        return fail(nullptr, B200UDE_EINVAL, "batch_create: unknown solver %d", d->solver);
+    if (d->sensealg != B200UDE_INTERPOLATING_ADJOINT && d->sensealg != B200UDE_DISCRETE_ADJOINT)
+        return fail(nullptr, B200UDE_EUNSUPPORTED, "batch_create: unknown sensealg %d", d->sensealg);
+    if (!(d->dt > 0) || d->n_steps < 1 || d->save_every < 1 || d->n_steps % d->save_every != 0)
+        return fail(nullptr, B200UDE_EINVAL, "batch_create: need dt>0, n_steps>=1, save_every>=1 dividing n_steps");
+    if (d->max_trajectories == 0 || d->max_trajectories > (1ull << 26))
+        return fail(nullptr, B200UDE_EINVAL, "batch_create: max_trajectories (the member capacity) out of range");
+    if (d->n_loss_weights != 0 && d->n_loss_weights != d->state_dim)
+        return fail(nullptr, B200UDE_EINVAL, "batch_create: n_loss_weights must be 0 or state_dim");
+    bool acts_ok = true;
+    for (int l = 0; l < d->n_layers; ++l) acts_ok = acts_ok && d->acts[l] >= 0 && d->acts[l] <= 2;
+    if (!acts_ok) return fail(nullptr, B200UDE_EINVAL, "batch_create: unknown activation");
+    const bool lv5 = d->model == B200UDE_MODEL_LV && d->state_dim == 2 && d->n_layers == 4 && d->widths[0] == 2 && d->widths[1] == 5 &&
+                     d->widths[2] == 5 && d->widths[3] == 5 && d->widths[4] == 2 && d->acts[3] == B200UDE_ACT_IDENTITY &&
+                     d->n_prefix >= 0 && d->n_prefix <= 2 && d->n_suffix == 0;
+    if (!lv5 || d->dtype != B200UDE_F32 || d->solver != B200UDE_TSIT5 || d->adaptive)
+        return fail(nullptr, B200UDE_EUNSUPPORTED,
+                          "batch_create: batched trainings have kernels for the LV 2-5-5-5-2 chain (identity output layer, 0..2 trainable "
+                          "rates), fp32, fixed-step Tsit5");
+    if (d->n_consts < 2) return fail(nullptr, B200UDE_EINVAL, "batch_create: the LV model needs n_consts >= 2");
+    int ndev = 0;
+    cudaError_t e = cudaGetDeviceCount(&ndev);
+    if (e != cudaSuccess || ndev == 0) return fail(nullptr, B200UDE_ENODEVICE, "batch_create: no CUDA device (%s)", cudaGetErrorString(e));
+    if (d->device < 0 || d->device >= ndev) return fail(nullptr, B200UDE_EINVAL, "batch_create: device %d of %d", d->device, ndev);
+    cudaDeviceProp prop;
+    e = cudaGetDeviceProperties(&prop, d->device);
+    if (e != cudaSuccess) return fail(nullptr, (int32_t)e, "batch_create: cudaGetDeviceProperties: %s", cudaGetErrorString(e));
+    if (prop.major != 10)
+        return fail(nullptr, B200UDE_ENODEVICE, "batch_create: device %d is sm_%d%d; this library carries sm_100a code only", d->device, prop.major, prop.minor);
+    e = cudaSetDevice(d->device);
+    if (e != cudaSuccess) return fail(nullptr, (int32_t)e, "batch_create: cudaSetDevice: %s", cudaGetErrorString(e));
+
+    b200ude_batch_handle *h = new (std::nothrow) b200ude_batch_handle();
+    if (!h) return fail(nullptr, B200UDE_ENOMEM, "batch_create: out of host memory");
+    h->desc = *d;
+    h->P = 87 + d->n_prefix;
+    h->n_save = d->n_steps / d->save_every + 1;
+    h->cap = (size_t)d->max_trajectories;
+    const size_t M = h->cap, P = (size_t)h->P, D = 2;
+    bool ok = cudaMalloc((void **)&h->d_theta, sizeof(float) * M * P) == cudaSuccess &&
+              cudaMalloc((void **)&h->d_m, sizeof(float) * M * P) == cudaSuccess &&
+              cudaMalloc((void **)&h->d_v, sizeof(float) * M * P) == cudaSuccess &&
+              cudaMalloc((void **)&h->d_ustep, sizeof(float) * ((size_t)d->n_steps + 1) * D * M) == cudaSuccess &&
+              cudaMalloc((void **)&h->d_dense, sizeof(float) * ((size_t)d->n_steps * 6 + 1) * D * M) == cudaSuccess &&
+              cudaMalloc((void **)&h->d_out, sizeof(float) * (size_t)h->n_save * D * M) == cudaSuccess &&
+              cudaMalloc((void **)&h->d_t, sizeof(int32_t) * M) == cudaSuccess &&
+              cudaMalloc((void **)&h->d_best, sizeof(float) * M * P) == cudaSuccess &&
+              cudaMalloc((void **)&h->d_best_loss, sizeof(float) * M) == cudaSuccess;
+    if (!ok) {
+        g_create_error = std::string("batch_create: device allocation failed: ") + cudaGetErrorString(cudaGetLastError());
+        b200ude_batch_destroy(h);
+        return B200UDE_ENOMEM;
+    }
+    h->tab.serial = ++g_serial;
+    h->tab.d_theta = nullptr;
+    h->tab.P = h->P;
+    for (int i = 0; i < 16; ++i) {
+        h->tab.consts[i] = i < d->n_consts ? (float)d->consts[i] : 0.0f;
+        h->tab.lossw[i] = d->n_loss_weights > 0 ? (i < d->n_loss_weights ? (float)d->loss_weights[i] : 0.0f) : 1.0f;
+    }
+    for (int i = 0; i < 8; ++i) h->tab.acts[i] = i < d->n_layers ? d->acts[i] : 0;
+    *out = h;
+    return B200UDE_OK;
+}
+
+void b200ude_batch_destroy(b200ude_batch_handle *h)
+{
+    if (!h) return;
+    cudaFree(h->d_theta); cudaFree(h->d_m); cudaFree(h->d_v);
+    cudaFree(h->d_ustep); cudaFree(h->d_dense); cudaFree(h->d_out);
+    cudaFree(h->d_t); cudaFree(h->d_best); cudaFree(h->d_best_loss);
+    delete h;
+}
+
+const char *b200ude_batch_last_error(const b200ude_batch_handle *h) { return h ? h->err.c_str() : g_create_error.c_str(); }
+
+size_t b200ude_batch_num_params(const b200ude_batch_handle *h) { return h ? (size_t)h->P : 0; }
+
+int32_t b200ude_batch_set_params(b200ude_batch_handle *h, const void *theta, size_t M, int32_t mem, void *stream)
+{
+    if (!h) return B200UDE_EINVAL;
+    if (!theta || M == 0 || M > h->cap) return fail(h, B200UDE_EINVAL, "batch_set_params: null theta or M=%zu outside (0, %zu]", M, h->cap);
+    CUDA_TRY(h, cudaSetDevice(h->desc.device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t bytes = sizeof(float) * M * (size_t)h->P;
+    CUDA_TRY(h, cudaMemcpyAsync(h->d_theta, theta, bytes, mem == B200UDE_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, st));
+    CUDA_TRY(h, cudaMemsetAsync(h->d_m, 0, sizeof(float) * h->cap * (size_t)h->P, st));
+    CUDA_TRY(h, cudaMemsetAsync(h->d_v, 0, sizeof(float) * h->cap * (size_t)h->P, st));
+    CUDA_TRY(h, cudaMemsetAsync(h->d_t, 0, sizeof(int32_t) * h->cap, st));
+    CUDA_TRY(h, cudaMemcpyAsync(h->d_best, h->d_theta, bytes, cudaMemcpyDeviceToDevice, st));
+    fill_kernel<<<(unsigned)std::min<size_t>((h->cap + 255) / 256, 1024), 256, 0, st>>>(h->d_best_loss, std::numeric_limits<float>::infinity(), h->cap);
+    CUDA_TRY(h, cudaGetLastError());
+    h->members = M;
+    return B200UDE_OK;
+}
+
+int32_t b200ude_batch_get_params(b200ude_batch_handle *h, void *theta, size_t M, int32_t mem, void *stream)
+{
+    if (!h) return B200UDE_EINVAL;
+    if (!theta || M == 0 || M > h->members) return fail(h, B200UDE_EINVAL, "batch_get_params: null theta or M=%zu outside (0, %zu]", M, h->members);
+    CUDA_TRY(h, cudaSetDevice(h->desc.device));
+    cudaStream_t st = (cudaStream_t)stream;
+    CUDA_TRY(h, cudaMemcpyAsync(theta, h->d_theta, sizeof(float) * M * (size_t)h->P,
+                                 mem == B200UDE_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, st));
+    if (mem != B200UDE_DEVICE) CUDA_TRY(h, cudaStreamSynchronize(st));
+    return B200UDE_OK;
+}
+
+int32_t b200ude_batch_forward(b200ude_batch_handle *h, const void *u0, size_t M, void *out, int32_t *status, void *stream)
+{
+    if (!h) return B200UDE_EINVAL;
+    BatchParams p;
+    int32_t rc = batch_prepare(h, M, u0, BATCH_FORWARD, p);
+    if (rc) return rc;
+    if (!out) return fail(h, B200UDE_EINVAL, "batch_forward: null out");
+    p.out = (float *)out;
+    p.status = status;
+    return batch_launch(h, p, (cudaStream_t)stream);
+}
+
+int32_t b200ude_batch_loss_gradient(b200ude_batch_handle *h, const void *u0, const void *data, size_t M, void *loss, void *grad,
+                                    int32_t *status, void *stream)
+{
+    if (!h) return B200UDE_EINVAL;
+    BatchParams p;
+    int32_t rc = batch_prepare(h, M, u0, BATCH_LOSS_GRAD, p);
+    if (rc) return rc;
+    if (!data || !loss || !grad) return fail(h, B200UDE_EINVAL, "batch_loss_gradient: null pointer");
+    p.data = (const float *)data;
+    p.loss = (float *)loss;
+    p.grad = (float *)grad;
+    p.status = status;
+    return batch_launch(h, p, (cudaStream_t)stream);
+}
+
+int32_t b200ude_batch_train_adam(b200ude_batch_handle *h, const b200ude_adam *o, const void *u0, const void *data, size_t M, int32_t iters,
+                                 void *loss_history, int32_t *status, void *stream)
+{
+    if (!h) return B200UDE_EINVAL;
+    if (!o || o->struct_size != sizeof(b200ude_adam)) return fail(h, B200UDE_EINVAL, "batch_train_adam: bad options struct");
+    if (!(o->eta > 0) || !(o->beta1 >= 0 && o->beta1 < 1) || !(o->beta2 >= 0 && o->beta2 < 1) || !(o->eps > 0))
+        return fail(h, B200UDE_EINVAL, "batch_train_adam: need eta > 0, 0 <= beta < 1, eps > 0");
+    if (!data || iters < 1) return fail(h, B200UDE_EINVAL, "batch_train_adam: null data or iters < 1");
+    BatchParams p;
+    int32_t rc = batch_prepare(h, M, u0, BATCH_TRAIN, p);
+    if (rc) return rc;
+    p.data = (const float *)data;
+    p.loss_history = (float *)loss_history;
+    p.status = status;
+    p.iters = iters;
+    p.eta = (float)o->eta; p.beta1 = (float)o->beta1; p.beta2 = (float)o->beta2; p.eps = (float)o->eps;
+    p.loss_scale = (float)(o->loss_scale == 0.0 ? 1.0 : o->loss_scale); p.l2_reg = (float)o->l2_reg;
+    return batch_launch(h, p, (cudaStream_t)stream);
+}
+
+int32_t b200ude_batch_get_best(b200ude_batch_handle *h, void *theta, void *loss, size_t M, int32_t mem, void *stream)
+{
+    if (!h) return B200UDE_EINVAL;
+    if (!theta || !loss || M == 0 || M > h->members)
+        return fail(h, B200UDE_EINVAL, "batch_get_best: null pointer or M=%zu outside (0, %zu]", M, h->members);
+    CUDA_TRY(h, cudaSetDevice(h->desc.device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const cudaMemcpyKind kind = mem == B200UDE_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
+    CUDA_TRY(h, cudaMemcpyAsync(theta, h->d_best, sizeof(float) * M * (size_t)h->P, kind, st));
+    CUDA_TRY(h, cudaMemcpyAsync(loss, h->d_best_loss, sizeof(float) * M, kind, st));
+    if (mem != B200UDE_DEVICE) CUDA_TRY(h, cudaStreamSynchronize(st));
     return B200UDE_OK;
 }
 

@@ -7,9 +7,6 @@
 
 namespace b200ude {
 
-template <int NP>
-using CfgLV5 = Cfg<MODEL_LV, 2, 2, 5, 3, 2, ACT_RUNTIME, NP, GRAD_LANE>;
-
 int adj_grid_lv5(int N) { return (N + ADJ_BLOCK_LANE - 1) / ADJ_BLOCK_LANE; }
 
 cudaError_t launch_fwd_lv5(int n_prefix, const Variant &, const ConstTables &t, const FwdParams &p, cudaStream_t st)

@@ -88,6 +88,28 @@ constexpr int FWD_BLOCK_LV32 = 32;  // packed LV32 forward: one warp (64 traject
 constexpr int ADJ_BLOCK_GEMM = 32;   // H=32 adjoint: one warp (64 trajectories) per CTA
 constexpr int ADJ_BLOCK_LANE = 128;  // small-chain adjoint
 
+// batched independent trainings (k_batch.cu, ude_batch.cuh): M members of the LV 2-5-5-5-2 UDE, one theta / gradient / ADAM state
+// per member, one member per thread.  Member-fastest layouts except theta.
+constexpr int BATCH_FORWARD = 0, BATCH_LOSS_GRAD = 1, BATCH_TRAIN = 2;
+constexpr int BATCH_BLOCK = 32;   // members per CTA: theta of the CTA in shared memory as [P][32] (11 KB at P = 89)
+struct BatchParams {
+    const float *u0;        // [D][M]
+    const float *data;      // [n_save][D][M]  (loss / gradient / train)
+    float *out;             // [n_save][D][M]  forward: the result; otherwise scratch
+    int32_t *status;        // [M]
+    float *theta;           // [M][P]: every member's theta contiguous (train writes the updated thetas back)
+    float *m, *v;           // [P][ldm] ADAM moments (train)
+    float *ustep, *dense;   // forward record [n_steps+1][D][M], [n_steps*6+1][D][M]
+    float *loss;            // [M]     (loss / gradient)
+    float *grad;            // [M][P]  (loss / gradient)
+    float *loss_history;    // [iters][M] or nullptr (train)
+    int32_t *t;             // [M] ADAM steps each member has taken (train; advanced only by the member's own updates)
+    float *best;            // [M][P] the member's best pre-update theta so far (train)
+    float *best_loss;       // [M] its loss (+inf: none yet)
+    int M, ldm, n_steps, save_every, mode, iters;
+    float dt, eta, beta1, beta2, eps, loss_scale, l2_reg;
+};
+
 // runtime shape of a UDE handled by the generic kernels (k_generic.cu)
 struct GenericShape {
     uint64_t serial;
@@ -118,6 +140,7 @@ cudaError_t launch_tanh_selftest(const float *x, float *y, size_t n, cudaStream_
 cudaError_t launch_fwd_lv32_adaptive(const Variant &, const ConstTables &, const FwdParams &, const AdaptiveGrid &, cudaStream_t);
 cudaError_t launch_adj_lv32_adaptive(const Variant &, const ConstTables &, const AdjParams &, const AdaptiveGrid &, cudaStream_t, int *rows_out);
 int adj_grid_lv5(int N);
+cudaError_t launch_batch(int n_prefix, bool discrete, const ConstTables &, const BatchParams &, cudaStream_t);
 cudaError_t launch_fwd_generic(const GenericShape &, const ConstTables &, const FwdParams &, cudaStream_t);
 cudaError_t launch_adj_generic(const GenericShape &, const ConstTables &, const AdjParams &, cudaStream_t, int *rows_out);
 int adj_rows_generic(int N);

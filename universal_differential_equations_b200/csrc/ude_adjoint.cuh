@@ -18,10 +18,19 @@
 namespace b200ude {
 
 // ---- pieces shared by both adjoint kernels -------------------------------------------------------
+// NC = true: the forward record and the data are read through the non-coherent read-only path (they are written by an earlier
+// launch).  A kernel that writes its own record in the same launch (the batched trainer, k_batch.cu) reads it with NC = false.
+template <bool NC>
+__device__ __forceinline__ float ld_rec(const float *a)
+{
+    if constexpr (NC) return __ldg(a);
+    else return *a;
+}
+
 // u(t_{s+1} - c_i dt) from the stored dense output of forward step s (Tsit5 free interpolant).
 // The k's are re-read per stage (L1-resident after the first touch) instead of being held in
 // registers across the stage evaluations.
-template <int D, int I>
+template <int D, int I, bool NC = true>
 __device__ __forceinline__ void interp_state(const AdjParams &p, int s, size_t n, size_t N, float dt, float (&x)[D])
 {
 #pragma unroll
@@ -30,8 +39,8 @@ __device__ __forceinline__ void interp_state(const AdjParams &p, int s, size_t n
 #pragma unroll
         for (int j = 0; j < 7; ++j)
             if (Tsit5::bw(I, j) != 0.0)
-                acc = fmaf((float)Tsit5::bw(I, j), __ldg(p.dense + ((size_t)(s * 6 + j) * D + c) * N + n), acc);
-        x[c] = fmaf(dt, acc, __ldg(p.ustep + ((size_t)s * D + c) * N + n));
+                acc = fmaf((float)Tsit5::bw(I, j), ld_rec<NC>(p.dense + ((size_t)(s * 6 + j) * D + c) * N + n), acc);
+        x[c] = fmaf(dt, acc, ld_rec<NC>(p.ustep + ((size_t)s * D + c) * N + n));
     }
 }
 
@@ -50,7 +59,7 @@ __device__ __forceinline__ void stage_arg(const float (&lam)[D], const float (&k
 
 // ---- discrete adjoint (exact gradient of the fixed-step Tsit5 scheme; what ForwardDiffSensitivity computes,
 // scenario_1.jl:86): stage argument g_i = u_n + dt sum_{j<i} a_ij k_j from the stored step start and stage derivatives ...
-template <int D, int I>
+template <int D, int I, bool NC = true>
 __device__ __forceinline__ void fwd_stage_state(const AdjParams &p, int s, size_t n, size_t N, float dt, float (&x)[D])
 {
 #pragma unroll
@@ -59,8 +68,8 @@ __device__ __forceinline__ void fwd_stage_state(const AdjParams &p, int s, size_
 #pragma unroll
         for (int j = 0; j < I; ++j)
             if (Tsit5::a(I, j) != 0.0)
-                acc = fmaf((float)Tsit5::a(I, j), __ldg(p.dense + ((size_t)(s * 6 + j) * D + c) * N + n), acc);
-        x[c] = fmaf(dt, acc, __ldg(p.ustep + ((size_t)s * D + c) * N + n));
+                acc = fmaf((float)Tsit5::a(I, j), ld_rec<NC>(p.dense + ((size_t)(s * 6 + j) * D + c) * N + n), acc);
+        x[c] = fmaf(dt, acc, ld_rec<NC>(p.ustep + ((size_t)s * D + c) * N + n));
     }
 }
 // ... and the cotangent of k_i: kbar_i = dt (b_i ubar_{n+1} + sum_{j>i} a_ji gbar_j), gbar_j = J_u(g_j)^T kbar_j of the later stages
@@ -78,7 +87,7 @@ __device__ __forceinline__ void disc_stage_cot(const float (&lam)[D], const floa
 }
 
 // lambda += dL/du(t_isave); with fused_l2 also accumulates the loss
-template <int D>
+template <int D, bool NC = true>
 __device__ __forceinline__ void loss_jump(const AdjParams &p, int isave, size_t n, size_t N, float (&lam)[D], float &loss)
 {
 #pragma unroll
@@ -87,12 +96,12 @@ __device__ __forceinline__ void loss_jump(const AdjParams &p, int isave, size_t 
         if (p.fused_l2) {
             // saved state i is the state at step i*save_every (the handle's own per-step store)
             const size_t idu = ((size_t)(isave * p.save_every) * D + c) * N + n;
-            const float r = __ldg(p.ustep + idu) - __ldg(p.cot + idx);
+            const float r = ld_rec<NC>(p.ustep + idu) - ld_rec<NC>(p.cot + idx);
             const float wgt = c_lossw[c];
             loss = fmaf(wgt * r, r, loss);
             lam[c] = fmaf(2.0f * wgt, r, lam[c]);
         } else {
-            lam[c] += __ldg(p.cot + idx);
+            lam[c] += ld_rec<NC>(p.cot + idx);
         }
     }
 }
@@ -100,37 +109,27 @@ __device__ __forceinline__ void loss_jump(const AdjParams &p, int isave, size_t 
 // =====================================================================================================
 // small chains: per-lane register accumulators
 // =====================================================================================================
-template <class C, int TM, class W, int BLOCK, int MINB, bool DISC = false>
-__global__ void __launch_bounds__(BLOCK, MINB) ude_adjoint_lane_kernel(AdjParams p)
+// Backward sweep of trajectory n: gacc[P] = its parameter gradient, lam = dL/du0, loss = its fused-L2 loss (fused_l2 only).
+// DISC selects the discrete adjoint (reverse accumulation through the stages) over the interpolating one.
+template <class C, int TM, class W, bool DISC, bool NC = true>
+__device__ __forceinline__ void lane_adjoint(const W &w, const AdjParams &p, size_t n, float (&gacc)[C::P], float (&lam)[C::D], float &loss)
 {
     static_assert(C::MODEL == MODEL_LV, "only the LV family has a kernel in this build");
     constexpr int D = C::D, H = C::H, NHID = C::NHID, DIN = C::DIN, DOUT = C::DOUT, P = C::P;
     constexpr bool NEED_PRE = (C::ACT != ACT_TANH && C::ACT != ACT_IDENTITY);
-    constexpr int NWARP = BLOCK / 32;
-    const W w = WeightStage<W>::load(p.theta, p.P);
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const size_t N = (size_t)p.N;
-    const int gid = blockIdx.x * BLOCK + threadIdx.x;
-    const bool live = gid < p.N;
-    const size_t n = live ? (size_t)gid : (size_t)(p.N - 1);
     const float dt = p.dt;
-
-    float gacc[P];
 #pragma unroll
     for (int q = 0; q < P; ++q) gacc[q] = 0.0f;
-
-    extern __shared__ __align__(16) unsigned char s_raw[];
-    constexpr int THETA_SMEM_FLOATS = WeightStage<W>::kSmem ? ((P + 3) / 4) * 4 : 0;
 
     float a1, a2;
     phys_rates<C>(w, a1, a2);
 
-    float lam[D];
-    float loss = 0.0f;
+    loss = 0.0f;
     const int n_save = p.n_steps / p.save_every + 1;
 #pragma unroll
     for (int c = 0; c < D; ++c) lam[c] = 0.0f;
-    loss_jump<D>(p, n_save - 1, n, N, lam, loss);
+    loss_jump<D, NC>(p, n_save - 1, n, N, lam, loss);
 
     auto stage_eval = [&](const float sc, const float (&x)[DIN], const float (&g)[D], float (&klI)[D]) {
         const float isc = 1.0f / sc;  // sc = dt*b_i: quadrature weight of this stage
@@ -222,14 +221,14 @@ __global__ void __launch_bounds__(BLOCK, MINB) ude_adjoint_lane_kernel(AdjParams
 #define B200UDE_LANE_STAGE(I)                                   \
     {                                                           \
         float x[DIN], g[D];                                     \
-        interp_state<D, I>(p, s, n, N, dt, x);                  \
+        interp_state<D, I, NC>(p, s, n, N, dt, x);              \
         stage_arg<D, I>(lam, kl, dt, g);                        \
         stage_eval(dt * (float)Tsit5::b(I), x, g, kl[I]);       \
     }
 #define B200UDE_LANE_DSTAGE(I)                                  \
     {                                                           \
         float x[DIN], kb[D];                                    \
-        fwd_stage_state<D, I>(p, s, n, N, dt, x);               \
+        fwd_stage_state<D, I, NC>(p, s, n, N, dt, x);           \
         disc_stage_cot<D, I>(lam, kl, dt, kb);                  \
         stage_eval(1.0f, x, kb, kl[I]);                         \
     }
@@ -266,8 +265,27 @@ __global__ void __launch_bounds__(BLOCK, MINB) ude_adjoint_lane_kernel(AdjParams
         }
 #undef B200UDE_LANE_STAGE
 #undef B200UDE_LANE_DSTAGE
-        if (s % p.save_every == 0) loss_jump<D>(p, s / p.save_every, n, N, lam, loss);
+        if (s % p.save_every == 0) loss_jump<D, NC>(p, s / p.save_every, n, N, lam, loss);
     }
+}
+
+template <class C, int TM, class W, int BLOCK, int MINB, bool DISC = false>
+__global__ void __launch_bounds__(BLOCK, MINB) ude_adjoint_lane_kernel(AdjParams p)
+{
+    constexpr int D = C::D, P = C::P;
+    constexpr int NWARP = BLOCK / 32;
+    const W w = WeightStage<W>::load(p.theta, p.P);
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const size_t N = (size_t)p.N;
+    const int gid = blockIdx.x * BLOCK + threadIdx.x;
+    const bool live = gid < p.N;
+    const size_t n = live ? (size_t)gid : (size_t)(p.N - 1);
+
+    extern __shared__ __align__(16) unsigned char s_raw[];
+    constexpr int THETA_SMEM_FLOATS = WeightStage<W>::kSmem ? ((P + 3) / 4) * 4 : 0;
+
+    float gacc[P], lam[D], loss;
+    lane_adjoint<C, TM, W, DISC>(w, p, n, gacc, lam, loss);
     if (p.grad_u0 && live) {
 #pragma unroll
         for (int c = 0; c < D; ++c) p.grad_u0[(size_t)c * N + n] = lam[c];

@@ -48,6 +48,16 @@ struct WSmem {  // shared-memory copy (bulk-copied once per CTA); compile-time o
     const float *p;
     __device__ __forceinline__ float operator()(int i) const { return p[i]; }
 };
+template <int STRIDE>
+struct WLane {  // one theta per lane in dynamic shared memory laid out [P][STRIDE]: lane l reads column l, so the warp's 32
+                // different weights at one index sit in 32 different banks (LDS with a compile-time offset i * STRIDE)
+    int lane;
+    __device__ __forceinline__ float operator()(int i) const
+    {
+        extern __shared__ __align__(16) float s_lane[];
+        return s_lane[i * STRIDE + lane];
+    }
+};
 
 // compile-time description of one UDE -----------------------------------------------------------
 template <int MODEL_, int D_, int DIN_, int H_, int NHID_, int DOUT_, int ACT_, int NPREFIX_, int GRAD_>
@@ -63,6 +73,11 @@ struct Cfg {
     static constexpr int P = OFF_BOUT + DOUT;  // (+ suffix for FKPP, none for LV/SEIR)
     static constexpr int JB = (H % 4 == 0) ? 4 : (H % 5 == 0 ? 5 : 1);  // output block of the H x H sweep
 };
+
+// the reference-shaped LV UDE: 2 -> 5 -> 5 -> 5 -> 2 chain, per-layer activations, NP trainable linear rates in front of the chain
+// (LotkaVolterra/scenario_1.jl:62-73, scenario_2.jl:79-98, hudson_bay.jl:77-91, loop_recoveries.jl:7-12)
+template <int NP>
+using CfgLV5 = Cfg<MODEL_LV, 2, 2, 5, 3, 2, ACT_RUNTIME, NP, GRAD_LANE>;
 
 // activations -------------------------------------------------------------------------------------
 // TM = 0: tanh(x) = 1 - 2/(2^(2 log2(e) x) + 1): MUFU.EX2 + MUFU.RCP, abs. error ~1e-7
@@ -268,27 +283,19 @@ struct WeightStage<WSmem> {
     }
 };
 
-template <class C, int T, int TM, class W, int BLOCK, int MINB>
-__global__ void __launch_bounds__(BLOCK, MINB) ude_forward_kernel(FwdParams p)
+// Whole fixed-step Tsit5 solve of trajectories n[0..T) from p.u0: writes the saved states, the per-step states and the dense
+// output (stores masked by live[]) and leaves the final state in us.
+template <class C, int T, int TM, class W>
+__device__ __forceinline__ void tsit5_record(const W &w, const FwdParams &p, const int (&n)[T], const bool (&live)[T], StateT<C::D, T> &us)
 {
     constexpr int D = C::D;
-    const W w = WeightStage<W>::load(p.theta, p.P);
-    const int NT = gridDim.x * BLOCK;
-    const int tid = blockIdx.x * BLOCK + threadIdx.x;
     const size_t N = (size_t)p.N;
-    int n[T];
-    bool live[T];
-    StateT<D, T> us;
     float (&u)[D][T] = us.v;
     float k[7][D][T];
 #pragma unroll
-    for (int t = 0; t < T; ++t) {
-        n[t] = tid + t * NT;
-        live[t] = n[t] < p.N;
-        if (!live[t]) n[t] = p.N - 1;  // duplicate work of the last trajectory; stores are masked
+    for (int t = 0; t < T; ++t)
 #pragma unroll
         for (int c = 0; c < D; ++c) u[c][t] = __ldg(p.u0 + (size_t)c * N + n[t]);
-    }
     const float dt = p.dt;
     auto store_state = [&](float *base, int row) {
 #pragma unroll
@@ -359,6 +366,26 @@ __global__ void __launch_bounds__(BLOCK, MINB) ude_forward_kernel(FwdParams p)
 #pragma unroll
             for (int t = 0; t < T; ++t) k[0][c][t] = k[6][c][t];
     }
+}
+
+template <class C, int T, int TM, class W, int BLOCK, int MINB>
+__global__ void __launch_bounds__(BLOCK, MINB) ude_forward_kernel(FwdParams p)
+{
+    constexpr int D = C::D;
+    const W w = WeightStage<W>::load(p.theta, p.P);
+    const int NT = gridDim.x * BLOCK;
+    const int tid = blockIdx.x * BLOCK + threadIdx.x;
+    int n[T];
+    bool live[T];
+#pragma unroll
+    for (int t = 0; t < T; ++t) {
+        n[t] = tid + t * NT;
+        live[t] = n[t] < p.N;
+        if (!live[t]) n[t] = p.N - 1;  // duplicate work of the last trajectory; stores are masked
+    }
+    StateT<D, T> us;
+    tsit5_record<C, T, TM>(w, p, n, live, us);
+    float (&u)[D][T] = us.v;
     if (p.status) {
 #pragma unroll
         for (int t = 0; t < T; ++t)

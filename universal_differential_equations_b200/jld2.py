@@ -3,7 +3,8 @@
 hudson_bay.jl:231-235) -- the data format either side of the training path (SURVEY.md section 8 f4).
 
 JLD2 0.1.x is an HDF5 container behind a 512-byte text header: superblock version 2, version-2 object headers ("OHDR", continued in
-"OCHK" blocks), hard links in link messages.  This module walks the root group's links and decodes the datasets whose element type is an
+"OCHK" blocks), hard links in link messages.  This module walks the root group's links -- and, for slash paths such as "17/X", the
+link messages of the groups on the way (`JLD2.Group`, loop_recoveries.jl's one group per run) -- and decodes the datasets whose element type is an
 IEEE float or an integer with contiguous or compact layout -- the arrays a training run needs (data X, time points t, loss histories).
 Julia structs (the `ODESolution`, `ComponentVector`, Lux chains ... that the same files hold as committed compound types with object
 references) are listed by `keys()`; `read_tree` follows a parameter container's references to its arrays, nothing else of a struct is
@@ -68,12 +69,30 @@ class JLD2File:
             raise ValueError(f"{path}: unsupported HDF5 superblock (need version 2 / 3 with 8-byte offsets and lengths)")
         self.base, _ext, _eof, root = struct.unpack_from("<QQQQ", b, i + 12)
         self.superblock_ok = lookup3(b[i:i + 44]) == struct.unpack_from("<I", b, i + 44)[0]
-        self.links = {}
-        for mtype, data in self._messages(root):
+        self.links = self._group_links(root)
+
+    def _group_links(self, addr):
+        """{name: object address} of the hard links in the link messages of the group object at addr."""
+        links = {}
+        for mtype, data in self._messages(addr):
             if mtype == 6:
-                name, addr = self._link(data)
-                if addr is not None:
-                    self.links[name] = addr
+                name, target = self._link(data)
+                if target is not None:
+                    links[name] = target
+        return links
+
+    def _addr(self, path):
+        """Object address of a root link or of a slash path through groups ("17/X"); KeyError when a component is missing."""
+        parts = [p for p in path.split("/") if p]
+        if not parts:
+            raise KeyError(path)
+        links = self.links
+        for i, part in enumerate(parts):
+            if part not in links:
+                raise KeyError(path)
+            if i == len(parts) - 1:
+                return links[part]
+            links = self._group_links(links[part])
 
     # ---- object headers (version 2) ----
     def _messages(self, addr):
@@ -126,7 +145,7 @@ class JLD2File:
 
     def header_bytes(self, name):
         """(bytes of the first chunk of the named object's header including its checksum, checksum valid?)"""
-        b, pos = self.blob, self.base + self.links[name]
+        b, pos = self.blob, self.base + self._addr(name)
         flags = b[pos + 5]
         q = pos + 6 + (16 if flags & 0x20 else 0) + (4 if flags & 0x10 else 0)
         n = 1 << (flags & 3)
@@ -134,11 +153,12 @@ class JLD2File:
         return b[pos:end + 4], lookup3(b[pos:end]) == struct.unpack_from("<I", b, end)[0]
 
     # ---- datasets ----
-    def keys(self):
-        return list(self.links)
+    def keys(self, group=None):
+        """Names of the root links, or of the links of the group at the slash path `group`."""
+        return list(self.links if group is None else self._group_links(self._addr(group)))
 
     def _describe(self, name):
-        return self._describe_at(self.links[name])
+        return self._describe_at(self._addr(name))
 
     def _describe_at(self, addr):
         dims = dtype = layout = None
@@ -169,9 +189,7 @@ class JLD2File:
     def read(self, name):
         """The dataset as a numpy array with the shape and element order the Julia array had (column-major data, HDF5 lists the
         dimensions slowest first, i.e. reversed)."""
-        if name not in self.links:
-            raise KeyError(name)
-        return self._read_at(self.links[name], name)
+        return self._read_at(self._addr(name), name)
 
     def _read_at(self, addr, name="<object>"):
         dims, dtype, layout = self._describe_at(addr)
@@ -197,7 +215,7 @@ class JLD2File:
         NamedTuple of layers, ...), depth first in field order.  JLD2 stores a struct as a fixed-size record whose array-valued fields are
         8-byte references to other objects of the file; this follows every field that is such a reference without decoding the committed
         compound type, so scalars that happen to look like an object address would be followed too -- meant for parameter containers."""
-        addr = self.links[name] if _addr is None else _addr
+        addr = self._addr(name) if _addr is None else _addr
         dims, dtype, layout = self._describe_at(addr)
         if dims is not None and dtype is not None and layout is not None:
             return [self._read_at(addr, name)]
@@ -212,7 +230,8 @@ class JLD2File:
 
 
 def load(path, *names):
-    """`load(path, "X", "t")` as in FileIO / JLD2: the named plain numeric datasets (all of them without names), as a dict."""
+    """`load(path, "X", "t")` as in FileIO / JLD2: the named plain numeric datasets (all of them without names), as a dict.
+    Names may be slash paths through groups ("17/X")."""
     f = JLD2File(path)
     names = names or [k for k in f.keys() if f.is_numeric(k)]
     return {k: f.read(k) for k in names}

@@ -301,6 +301,38 @@ def _stream_ptr(device):
     return C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
 
 
+def _desc(f, device_index, dtype, alg, sensealg, t0, dt, n_steps, save_every, loss_weights, max_trajectories):
+    """struct b200ude_desc of a UDE form on a fixed grid."""
+    d = _lib.Desc()
+    d.struct_size = C.sizeof(_lib.Desc)
+    d.device = device_index
+    d.dtype = _lib.F64 if dtype == torch.float64 else _lib.F32
+    d.model = f.model
+    d.state_dim = f.state_dim
+    chain = f.chain
+    d.n_layers = len(chain.layers)
+    for i, w in enumerate(chain.widths):
+        d.widths[i] = w
+    for i, a in enumerate(chain.acts):
+        d.acts[i] = _ACT_CODE[a]
+    d.n_prefix = getattr(f, "trainable_rates", 0)
+    d.n_suffix = getattr(f, "n_suffix", 0)
+    cs = f.consts()
+    d.n_consts = len(cs)
+    for i, c in enumerate(cs):
+        d.consts[i] = c
+    d.solver = alg.code
+    d.n_stages = alg.n_stages(float(dt)) if isinstance(alg, RKC2) else 0
+    d.sensealg = sensealg.code
+    d.t0, d.dt, d.n_steps, d.save_every = t0, dt, n_steps, save_every
+    if loss_weights is not None:
+        d.n_loss_weights = len(loss_weights)
+        for i, w in enumerate(loss_weights):
+            d.loss_weights[i] = float(w)
+    d.max_trajectories = int(max_trajectories)
+    return d
+
+
 class UDESolver:
     """One C-ABI handle: a UDE form, a fixed Tsit5 grid and a capacity of trajectories."""
 
@@ -316,36 +348,10 @@ class UDESolver:
         self.device = torch.device("cuda", torch.cuda.current_device() if device is None else torch.device(device).index or 0)
         self.f = f
         self.n_steps, self.save_every, self.dt, self.t0 = int(n_steps), int(save_every), float(dt), float(t0)
-        d = _lib.Desc()
-        d.struct_size = C.sizeof(_lib.Desc)
-        d.device = self.device.index
         if dtype not in (torch.float32, torch.float64):
             raise TypeError("dtype must be torch.float32 or torch.float64")
         self.dtype = dtype
-        d.dtype = _lib.F64 if dtype == torch.float64 else _lib.F32
-        d.model = f.model
-        d.state_dim = f.state_dim
-        chain = f.chain
-        d.n_layers = len(chain.layers)
-        for i, w in enumerate(chain.widths):
-            d.widths[i] = w
-        for i, a in enumerate(chain.acts):
-            d.acts[i] = _ACT_CODE[a]
-        d.n_prefix = getattr(f, "trainable_rates", 0)
-        d.n_suffix = getattr(f, "n_suffix", 0)
-        cs = f.consts()
-        d.n_consts = len(cs)
-        for i, c in enumerate(cs):
-            d.consts[i] = c
-        d.solver = alg.code
-        d.n_stages = alg.n_stages(float(dt)) if isinstance(alg, RKC2) else 0
-        d.sensealg = sensealg.code
-        d.t0, d.dt, d.n_steps, d.save_every = self.t0, self.dt, self.n_steps, self.save_every
-        if loss_weights is not None:
-            d.n_loss_weights = len(loss_weights)
-            for i, w in enumerate(loss_weights):
-                d.loss_weights[i] = float(w)
-        d.max_trajectories = int(max_trajectories)
+        d = _desc(f, self.device.index, dtype, alg, sensealg, self.t0, self.dt, self.n_steps, self.save_every, loss_weights, max_trajectories)
         d.flags = _lib.FLAG_APPROX_TANH if approx_tanh else 0
         # adaptive = true: OrdinaryDiffEq's defaults abstol = 1e-6, reltol = 1e-3 when the kwargs are omitted (Fisher-KPP-CNN.jl:136)
         d.adaptive = 1 if adaptive else 0
@@ -511,6 +517,122 @@ class UDESolver:
         _lib.check(self._h, self._L.b200ude_train_adam(self._h, C.byref(a), u0.data_ptr(), data.data_ptr(), u0.shape[1], iters,
                                                      loss_history.data_ptr(), _stream_ptr(self.device)))
         return loss_history
+
+
+class UDEBatchSolver:
+    """M independent trainings at once (b200ude_batch_*): the batch counterpart of UDESolver for the reference's LV UDE with the
+    2-5-5-5-2 chain, fixed-step Tsit5, fp32.  Every member has its own theta, u0, data, gradient and ADAM moments; one trajectory per
+    member.  The device counterpart of run_loops.jl:55-62's loop over recover_dynamics.  Arrays: theta / grad [M, P] (row n = member
+    n's flat theta in the reference's order), u0 [d, M], data / out [n_save, d, M], loss / status [M], loss history [iters, M]."""
+
+    def __init__(self, f, t0, dt, n_steps, save_every=1, max_members=1, device=None, loss_weights=None, sensealg=None):
+        sensealg = sensealg or InterpolatingAdjoint()
+        if not isinstance(sensealg, (InterpolatingAdjoint, ForwardDiffSensitivity)):
+            raise TypeError(f"unsupported sensealg {sensealg!r}")
+        if not torch.cuda.is_available():
+            raise RuntimeError("b200ude needs a CUDA device (sm_100a); there is no CPU fallback")
+        self.device = torch.device("cuda", torch.cuda.current_device() if device is None else torch.device(device).index or 0)
+        self.f = f
+        self.n_steps, self.save_every, self.dt, self.t0 = int(n_steps), int(save_every), float(dt), float(t0)
+        d = _desc(f, self.device.index, torch.float32, Tsit5(), sensealg, self.t0, self.dt, self.n_steps, self.save_every, loss_weights,
+                  max_members)
+        self._L = _lib.lib()
+        h = C.c_void_p()
+        rc = self._L.b200ude_batch_create(C.byref(d), C.byref(h))
+        if rc != 0:
+            raise _lib.B200UDEError(rc, (self._L.b200ude_batch_last_error(None) or b"").decode())
+        self._h = h
+        self.P = int(self._L.b200ude_batch_num_params(h))
+        self.n_save = self.n_steps // self.save_every + 1
+        self.d = f.state_dim
+        self.capacity = int(max_members)
+        self.members = 0
+
+    def close(self):
+        if getattr(self, "_h", None):
+            self._L.b200ude_batch_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def _check(self, rc):
+        _lib.check_batch(self._h, rc)
+
+    def _inputs(self, u0, data=None):
+        """Checks u0 [d, M] (and data [n_save, d, M]): CUDA float32 on the solver's device, M within the members set; returns them
+        contiguous with M."""
+        for name, a in (("u0", u0), ("data", data)):
+            if a is None:
+                continue
+            if not isinstance(a, torch.Tensor) or not a.is_cuda or a.dtype != torch.float32 or a.device != self.device:
+                raise TypeError(f"{name} must be a float32 CUDA tensor on {self.device}")
+        if u0.dim() != 2 or u0.shape[0] != self.d:
+            raise ValueError(f"u0 must be [{self.d}, M], got {tuple(u0.shape)}")
+        M = u0.shape[1]
+        if not 0 < M <= self.members:
+            raise ValueError(f"M = {M} members, but set_params stored {self.members}")
+        if data is not None and tuple(data.shape) != (self.n_save, self.d, M):
+            raise ValueError(f"data must be [{self.n_save}, {self.d}, {M}], got {tuple(data.shape)}")
+        return u0.contiguous(), (data.contiguous() if data is not None else None), M
+
+    def set_params(self, theta):
+        """theta [M, P] (host or device, float32) -> members 0..M-1; zeroes their ADAM state."""
+        theta = torch.as_tensor(theta).detach().to(torch.float32).contiguous()
+        if theta.dim() != 2 or theta.shape[1] != self.P or not 0 < theta.shape[0] <= self.capacity:
+            raise ValueError(f"theta must be [M, {self.P}] with 0 < M <= {self.capacity}")
+        if theta.is_cuda and theta.device != self.device:
+            raise ValueError(f"theta is on {theta.device}, the solver on {self.device}")
+        mem = _lib.DEVICE if theta.is_cuda else _lib.HOST
+        self._check(self._L.b200ude_batch_set_params(self._h, theta.data_ptr(), theta.shape[0], mem, _stream_ptr(self.device)))
+        self._theta_keepalive = theta
+        self.members = theta.shape[0]
+
+    def get_params(self, M=None) -> torch.Tensor:
+        """The current thetas of members 0..M-1 [M, P]."""
+        M = self.members if M is None else M
+        th = torch.empty((M, self.P), device=self.device, dtype=torch.float32)
+        self._check(self._L.b200ude_batch_get_params(self._h, th.data_ptr(), M, _lib.DEVICE, _stream_ptr(self.device)))
+        return th
+
+    def get_best(self, M=None):
+        """Every member's best pre-update theta since set_params [M, P] and its loss [M] (+inf when it recorded no finite loss)."""
+        M = self.members if M is None else M
+        th = torch.empty((M, self.P), device=self.device, dtype=torch.float32)
+        loss = torch.empty(M, device=self.device, dtype=torch.float32)
+        self._check(self._L.b200ude_batch_get_best(self._h, th.data_ptr(), loss.data_ptr(), M, _lib.DEVICE, _stream_ptr(self.device)))
+        return th, loss
+
+    def forward(self, u0: torch.Tensor):
+        """u0 [d, M] -> (out [n_save, d, M], status [M])."""
+        u0, _, M = self._inputs(u0)
+        out = torch.empty((self.n_save, self.d, M), device=self.device, dtype=torch.float32)
+        status = torch.empty(M, device=self.device, dtype=torch.int32)
+        self._check(self._L.b200ude_batch_forward(self._h, u0.data_ptr(), M, out.data_ptr(), status.data_ptr(), _stream_ptr(self.device)))
+        return out, status
+
+    def loss_gradient(self, u0: torch.Tensor, data: torch.Tensor):
+        """Per-member fused L2 loss and gradient: (loss [M], grad [M, P], status [M])."""
+        u0, data, M = self._inputs(u0, data)
+        loss = torch.empty(M, device=self.device, dtype=torch.float32)
+        grad = torch.empty((M, self.P), device=self.device, dtype=torch.float32)
+        status = torch.empty(M, device=self.device, dtype=torch.int32)
+        self._check(self._L.b200ude_batch_loss_gradient(self._h, u0.data_ptr(), data.data_ptr(), M, loss.data_ptr(), grad.data_ptr(),
+                                                        status.data_ptr(), _stream_ptr(self.device)))
+        return loss, grad, status
+
+    def train_adam(self, opt, u0: torch.Tensor, data: torch.Tensor, iters: int, loss_scale=1.0, l2_reg=0.0):
+        """`iters` ADAM iterations of every member in one launch: (loss history [iters, M] at the pre-update thetas, status [M])."""
+        u0, data, M = self._inputs(u0, data)
+        a = UDESolver._adam_struct(opt, loss_scale, l2_reg)
+        hist = torch.empty((iters, M), device=self.device, dtype=torch.float32)
+        status = torch.empty(M, device=self.device, dtype=torch.int32)
+        self._check(self._L.b200ude_batch_train_adam(self._h, C.byref(a), u0.data_ptr(), data.data_ptr(), M, iters, hist.data_ptr(),
+                                                     status.data_ptr(), _stream_ptr(self.device)))
+        return hist, status
 
 
 class _SolveFn(torch.autograd.Function):
@@ -747,3 +869,25 @@ def sciml_train_l2(solver: "UDESolver", theta0, u0: torch.Tensor, data: torch.Te
     res = TrainResult(best_th, best, it)
     res.final = solver.get_params()
     return res
+
+
+@dataclass
+class BatchTrainResult:
+    minimizers: torch.Tensor   # [M, P]: every member's best pre-update theta (sciml_train's minimizer; theta0 if no finite loss)
+    minimum: torch.Tensor      # [M]: its loss (+inf: no finite loss)
+    losses: torch.Tensor       # [maxiters, M]: loss at the pre-update theta of each iteration (NaN after a member stopped)
+    status: torch.Tensor       # [M]: 0, or B200UDE_TRAJ_NONFINITE for a member whose state, loss or gradient turned non-finite
+    final: torch.Tensor        # [M, P]: every member's theta after its last update (a stopped member: its last finite theta)
+
+
+def sciml_train_batch(solver: "UDEBatchSolver", theta0, u0: torch.Tensor, data: torch.Tensor, opt: "ADAM", maxiters: int = 100,
+                      loss_scale: float = 1.0, l2_reg: float = 0.0) -> BatchTrainResult:
+    """sciml_train(loss, theta, ADAM(eta); maxiters) for M independent problems at once -- the ADAM phase of every run of
+    run_loops.jl:55-62 (loop_recoveries.jl:71-77) in one device call.  theta0 [M, P], u0 [d, M], data [n_save, d, M]; the loss is
+    loss_scale * sum w (u - data)^2 + l2_reg * sum theta[n_prefix:]^2 per member (the loop: l2_reg = 1e-4 / P).  As sciml_train, every
+    member's minimizer is the theta of its lowest recorded loss -- what loop_recoveries.jl:78-84 hands to BFGS; `.final` is the last
+    iterate."""
+    solver.set_params(theta0)
+    losses, status = solver.train_adam(opt, u0, data, maxiters, loss_scale, l2_reg)
+    best, minimum = solver.get_best()
+    return BatchTrainResult(best, minimum, losses, status, solver.get_params())
